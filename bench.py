@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- audio-seconds separated per second.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path (STFT -> encoder/decoder -> soft mask + cross-fade ->
@@ -23,6 +23,10 @@ iSTFT/OLA) over one batch of synthetic mono 44.1 kHz mixtures per GPU.  `--confi
 `cpu_baseline`: the float64 numpy oracle (the restated reference path) on a bounded sample.
 `--impl reference` times that CPU path on the host cores this process may really use (the reference itself --
 Python 2 + Theano 0.9 + Lasagne -- cannot be installed here; see DESIGN.md).
+`--dump-outputs DIR` writes the stems the last timed step computed to DIR/stems.npy (float32), so that two builds
+can be compared output for output: the inputs depend on the command line only.  Stems of more than
+DUMP_SAMPLES values (the default workload's are 4 GB) are written as the values at a fixed seeded sample of
+positions instead (`dump_positions`).
 """
 import argparse
 import json
@@ -38,6 +42,7 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 SR = 44100
+DUMP_SAMPLES = 8_000_000          # float32 values in a sampled dump: 32 MB
 METRIC = "audio_seconds_separated_per_second"
 _emit = print
 UNIT = "audio-s/s"
@@ -75,8 +80,12 @@ def parse_args():
                     help="live: one ncu pass over one clip after the timing (dram bytes of the dominant kernel)")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--ref-clip-seconds", type=float, default=None, help="reference arm: clip length (default: sized to the run)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the stems of the last timed step (or a fixed sample of them) to DIR/stems.npy")
     ap.add_argument("--traffic-probe", action="store_true", help=argparse.SUPPRESS)
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[a.config])
     if a.frame_size is not None:
         if cfg["arch"] != "dsd":
@@ -419,6 +428,23 @@ def make_separator(cfg, params, device):
                      patcher=cfg["patcher"], scale_factor=cfg["scale"], feat_size=cfg["N"] // 2 + 1, device=device)
 
 
+def dump_positions(total):
+    """Sorted flat positions of the sampled dump of `total` output values: the same for the same shape."""
+    import numpy as np
+    return np.unique(np.random.default_rng(0).integers(0, total, size=DUMP_SAMPLES))
+
+
+def dump_outputs(path, outs):
+    """outs: float32 cuda [clips, sources, samples], the stems as a caller of the timed path receives them."""
+    import numpy as np
+    import torch
+    if outs.numel() > DUMP_SAMPLES:
+        idx = torch.from_numpy(dump_positions(outs.numel())).to(outs.device)
+        outs = outs.reshape(-1)[idx]
+    os.makedirs(os.path.dirname(path) or ".", exist_ok=True)
+    np.save(path, outs.cpu().numpy())
+
+
 def parity_check(args, sep):
     """One clip of this very run against stems the float64 oracle produced for it (committed fixture made by
     tools/make_bench_check.py).  Plain 1e-4 per stem; the few time-frequency bins the ORACLE flagged as
@@ -556,6 +582,8 @@ def run_ours(args):
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     launches = sum(w.ctx.launch_count() for w in dworkers) - launches0
     clocks = sampler.stop(t_host0, t_host1)
+    if args.dump_outputs:
+        dump_outputs(os.path.join(args.dump_outputs, "stems.npy" if world == 1 else "stems_rank%d.npy" % rank), outs)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms = float(ms.item())

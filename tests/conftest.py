@@ -13,5 +13,5 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    import numpy as np
-    return np.load(os.path.join(ROOT, "tests", "golden", "dsp_golden.npz"))
+    import dspgolden
+    return dspgolden.load(os.path.join(ROOT, "tests", "golden", "dsp_golden.npz"))

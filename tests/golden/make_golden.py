@@ -5,7 +5,8 @@ Run in the build container only (needs /root/reference).  The reference files ar
 (print statements) and cannot be imported, but the hot-path functions themselves are valid
 Python 3: their source text is sliced out of the reference files at run time (nothing is
 copied into this repo), exec'd with numpy in scope, and run on seeded inputs.  The outputs
-pin oracle/dsp.py and oracle/patch.py (tests/test_oracle_golden.py).
+pin oracle/dsp.py and oracle/patch.py (tests/test_oracle_golden.py); tests/dspgolden.py makes the
+inputs and says how dsp_golden.npz stores the outputs.
 
 The network (Theano/Lasagne) cannot be executed here -> no golden for it (parity unpinned).
 """
@@ -16,6 +17,8 @@ import numpy as np
 
 REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE))
+import dspgolden  # noqa: E402
 
 
 def grab(path, names):
@@ -30,7 +33,6 @@ def grab(path, names):
 
 
 def main():
-    rng = np.random.default_rng(20260923)
     tr = grab("transform.py", ["sinebell", "stft_norm", "istft_norm"])
     sd = grab("examples/dsd100/separate_dsd.py",
               ["sinebell", "stft_norm", "istft_norm", "compute_file", "compute_inverse",
@@ -39,51 +41,50 @@ def main():
     ut = grab("util.py", ["generate_overlapadd", "overlapadd_multi"])
 
     out = {}
+    stream = iter(range(2000, 3000))        # sample positions of each stored output
+
+    def keep(key, a):
+        out.update(dspgolden.record(key, a, next(stream)))
     # --- STFT / iSTFT (transform.py) for the three frame sizes and three windows
     from scipy.signal import windows
-    cases = [(1024, 512, "hanning", 5000), (2048, 512, "hanning", 7013), (4096, 512, "blackmanharris", 9001),
-             (1024, 256, "sinebell", 3000), (1024, 512, "hanning", 512), (1024, 512, "hanning", 1)]
-    for ci, (N, H, wname, L) in enumerate(cases):
+    for ci, (N, H, wname, L) in enumerate(dspgolden.STFT_CASES):
         w = {"hanning": np.hanning, "blackmanharris": windows.blackmanharris,
              "sinebell": tr["sinebell"]}[wname](N)
-        x = rng.standard_normal(L) * 0.1
+        x, Z = dspgolden.stft_inputs(ci)
         X = tr["stft_norm"](x, window=w, hopsize=float(H), nfft=float(N), fs=44100.0)
-        y = tr["istft_norm"](X, window=w, analysisWindow=w, hopsize=float(H), nfft=float(N))
-        # a non-Hermitian-consistent spectrum exercises irfft's "ignore imag of DC/Nyquist"
-        Z = X * (0.5 + rng.random(X.shape)) * np.exp(1j * rng.standard_normal(X.shape))
-        y2 = tr["istft_norm"](Z, window=w, analysisWindow=w, hopsize=float(H), nfft=float(N))
-        out.update({"stft%d_x" % ci: x, "stft%d_w" % ci: w, "stft%d_NH" % ci: np.array([N, H]),
-                    "stft%d_X" % ci: X, "stft%d_y" % ci: y, "stft%d_Z" % ci: Z, "stft%d_y2" % ci: y2})
-    out["n_stft"] = np.array(len(cases))
+        assert X.shape == Z.shape
+        out.update({"stft%d_w" % ci: w, "stft%d_NH" % ci: np.array([N, H])})
+        keep("stft%d_X" % ci, X)
+        keep("stft%d_y" % ci, tr["istft_norm"](X, window=w, analysisWindow=w, hopsize=float(H), nfft=float(N)))
+        keep("stft%d_y2" % ci, tr["istft_norm"](Z, window=w, analysisWindow=w, hopsize=float(H), nfft=float(N)))
+    out["n_stft"] = np.array(len(dspgolden.STFT_CASES))
     # --- compute_file / compute_inverse of the stand-alone script (hanning 1024/512 defaults)
-    x = rng.standard_normal(6000) * 0.1
-    mag, ph = sd["compute_file"](x, phase=True)
-    out.update({"cf_x": x, "cf_mag": mag, "cf_ph": ph,
-                "cf_inv": sd["compute_inverse"](mag * 0.7, ph)})
+    mag, ph = sd["compute_file"](dspgolden.cf_input(), phase=True)
+    keep("cf_mag", mag)
+    keep("cf_ph", ph)
+    keep("cf_inv", sd["compute_inverse"](mag * 0.7, ph))
     # --- patchers + cross-fade
-    pc = [(100, 17, 30, 25, 32), (64, 9, 30, 20, 8), (30, 5, 30, 25, 32), (31, 5, 30, 25, 4), (203, 7, 20, 15, 16)]
-    for ci, (T, F, tc, ov, bs) in enumerate(pc):
-        m = rng.random((T, F))
+    for ci, (T, F, tc, ov, bs) in enumerate(dspgolden.PATCH_CASES):
+        m = dspgolden.patch_input(ci)
         fb, n = sd["generate_overlapadd"](m, input_size=F, time_context=tc, overlap=ov, batch_size=bs)
         if n:
             fb[int((n - 1) / bs), int((n - 1) % bs) + 1:] = 0   # np.empty tail -> deterministic
         fbu, nu = ut["generate_overlapadd"](m, input_size=F, time_context=tc, overlap=ov, batch_size=bs)
-        out.update({"pat%d_m" % ci: m, "pat%d_cfg" % ci: np.array([tc, ov, bs]),
-                    "pat%d_fb" % ci: fb, "pat%d_n" % ci: np.array(n),
-                    "pat%d_fbu" % ci: fbu, "pat%d_nu" % ci: np.array(nu)})
+        out.update({"pat%d_cfg" % ci: np.array([tc, ov, bs]), "pat%d_n" % ci: np.array(n), "pat%d_nu" % ci: np.array(nu)})
+        keep("pat%d_fb" % ci, fb)
+        keep("pat%d_fbu" % ci, fbu)
         if n:
-            nb = fb.shape[0]
-            pred = rng.random((nb, 4, bs, 1, tc, F))
-            out["pat%d_pred" % ci] = pred
-            out["pat%d_sep" % ci] = sd["overlapadd_multi"](pred, fb, n, overlap=ov)
-            out["pat%d_sepu" % ci] = ut["overlapadd_multi"](pred, fb, n, overlap=ov)
+            pred = dspgolden.patch_pred(ci, n)
+            assert pred.shape[0] == fb.shape[0]
+            keep("pat%d_sep" % ci, sd["overlapadd_multi"](pred, fb, n, overlap=ov))
+            keep("pat%d_sepu" % ci, ut["overlapadd_multi"](pred, fb, n, overlap=ov))
             s1, s2 = ik["overlapadd"](pred[:, :2], fb, n, overlap=ov)
-            out["pat%d_sep2" % ci] = np.stack([s1, s2])
-    out["n_pat"] = np.array(len(pc))
+            keep("pat%d_sep2" % ci, np.stack([s1, s2]))
+    out["n_pat"] = np.array(len(dspgolden.PATCH_CASES))
     # 3-D (channel) input through util's patcher (score-informed path)
-    m3 = rng.random((4, 57, 11))
-    fb3, n3 = ut["generate_overlapadd"](m3, input_size=11, time_context=30, overlap=25, batch_size=8)
-    out.update({"pat3d_m": m3, "pat3d_fb": fb3, "pat3d_n": np.array(n3)})
+    fb3, n3 = ut["generate_overlapadd"](dspgolden.pat3d_input(), input_size=11, time_context=30, overlap=25, batch_size=8)
+    out["pat3d_n"] = np.array(n3)
+    keep("pat3d_fb", fb3)
     np.savez_compressed(os.path.join(HERE, "dsp_golden.npz"), **out)
     print("wrote", os.path.join(HERE, "dsp_golden.npz"), len(out), "arrays")
 

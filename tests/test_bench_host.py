@@ -63,6 +63,30 @@ def test_bench_check_fixtures_are_consistent():
         assert g["S_or_flag"].shape == (bench.CONFIGS[name]["nsrc"], g["flag_t"].size)
 
 
+def test_steps_must_be_positive(monkeypatch):
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.parse_args()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "7", "--dump-outputs", "out"])
+    a = bench.parse_args()
+    assert a.steps == 7 and a.dump_outputs == "out"
+
+
+def test_dump_outputs_whole_or_a_fixed_sample(tmp_path):
+    import torch
+    small = torch.arange(24, dtype=torch.float32).reshape(2, 3, 4)
+    bench.dump_outputs(str(tmp_path / "a" / "stems.npy"), small)
+    np.testing.assert_array_equal(np.load(str(tmp_path / "a" / "stems.npy")), small.numpy())
+    big = torch.rand((2, 4, 1500000), generator=torch.Generator().manual_seed(0))
+    pos = bench.dump_positions(big.numel())
+    assert np.array_equal(pos, bench.dump_positions(big.numel())) and np.all(np.diff(pos) > 0)
+    assert 0 <= pos[0] and pos[-1] < big.numel()
+    bench.dump_outputs(str(tmp_path / "b" / "stems.npy"), big)
+    got = np.load(str(tmp_path / "b" / "stems.npy"))
+    assert got.dtype == np.float32 and got.nbytes <= 64 * 10 ** 6
+    np.testing.assert_array_equal(got, big.numpy().reshape(-1)[pos])
+
+
 def test_both_arms_print_the_same_config(monkeypatch):
     """`config` is a function of the command line and WORLD_SIZE only: the reference arm (launched by the driver
     with the same flags, torchrun included) names the same workload as this arm; its bounded sample lives elsewhere."""

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 from deepconvsep_b200 import util
+from dspgolden import check
 from oracle import patch
 
 
@@ -40,11 +41,13 @@ def test_golden_patchers(golden):
         tc, ov, bs = (int(v) for v in g["pat%d_cfg" % ci])
         m = g["pat%d_m" % ci]
         fb, n = util.generate_overlapadd_standalone(m, m.shape[1], tc, ov, bs)
-        assert n == int(g["pat%d_n" % ci]) and np.array_equal(fb, g["pat%d_fb" % ci])
+        assert n == int(g["pat%d_n" % ci])
+        check(g, "pat%d_fb" % ci, fb)
         fbu, nu = util.generate_overlapadd(m, m.shape[1], tc, ov, bs)
-        assert nu == int(g["pat%d_nu" % ci]) and np.array_equal(fbu, g["pat%d_fbu" % ci])
+        assert nu == int(g["pat%d_nu" % ci])
+        check(g, "pat%d_fbu" % ci, fbu)
         if n:
-            assert np.array_equal(util.overlapadd_multi(g["pat%d_pred" % ci], fb, n, ov), g["pat%d_sep" % ci])
+            check(g, "pat%d_sep" % ci, util.overlapadd_multi(g["pat%d_pred" % ci], fb, n, ov))
 
 
 def test_wav_helpers_and_tensor_dump(tmp_path):

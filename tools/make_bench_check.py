@@ -21,7 +21,7 @@ sys.path.insert(0, ROOT)
 import bench  # noqa: E402
 from oracle import dsp, pipeline  # noqa: E402
 
-SECONDS = {"dsd2048": 1.5, "dsd1024": 1.5, "ikala": 1.5, "bach10": 1.0, "bach10_score": 1.0}
+SECONDS = {"dsd2048": 1.0, "dsd1024": 1.0, "ikala": 1.5, "bach10": 1.0, "bach10_score": 1.0}   # each fixture under 1 MB
 
 
 def make(name):
